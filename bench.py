@@ -16,6 +16,7 @@ section 3), synthetic DTLZ2-shaped training targets.  One *step* = one generatio
   python bench.py --gpus N --steps K --warmup W            # this build (one process per GPU under torchrun for N > 1)
   python bench.py --impl reference ...                     # CPU arm: the UNMODIFIED reference (baseline/_ref) on the host
                                                            # cores at a bounded population; the oracle port if it is absent
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's population as DIR/<name>.npy
 
 Extra legs printed in the same JSON line (rank 0, N = 1): `hv_contrib` (the second half of BASELINE's metric: expected-HV-
 improvement contributions / s, A17) and `sort_hv` (rank + truncation + hypervolume on SURVEY section 8d's three objective
@@ -23,10 +24,12 @@ sets: GP-predicted, uniform, near-single-front sphere).
 """
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
@@ -97,16 +100,23 @@ class ClockSampler:
         self.device = device
         self.proc = None
         self.t0 = self.t1 = None
-        self.path = os.path.join(ROOT, "gpurun_out", f"clocks_bench_{os.getpid()}.csv")
 
     def start(self):
         try:
-            os.makedirs(os.path.dirname(self.path), exist_ok=True)
-            self.f = open(self.path, "w")
+            self.f = tempfile.TemporaryFile(mode="w+")  # the benchmark writes nothing into the tree (it may be read-only)
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "50", "-i", str(self.device)],
                                          stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self._terminate)  # no sampler outlives a run that fails before stop()
         except Exception:
             self.proc = None
+
+    def _terminate(self):
+        if self.proc is not None and self.proc.poll() is None:
+            self.proc.terminate()
+            try:
+                self.proc.wait(timeout=5)
+            except Exception:
+                self.proc.kill()
 
     def mark_begin(self):
         import datetime
@@ -125,15 +135,13 @@ class ClockSampler:
         if self.proc is None:
             return out
         time.sleep(0.06)  # one more sampling period so that a row stamped inside the region is flushed
-        self.proc.terminate()
-        try:
-            self.proc.wait(timeout=5)
-        except Exception:
-            self.proc.kill()
+        self._terminate()
+        self.f.seek(0)
+        lines = self.f.readlines()
         self.f.close()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         rows = []
-        for line in open(self.path):
+        for line in lines:
             parts = [p.strip() for p in line.split(",")]
             if len(parts) < 10:
                 continue
@@ -379,6 +387,23 @@ class ResidentStep:
         return P
 
 
+def dump_outputs(out_dir, rs, limit_bytes=64 << 20, seed=0):
+    """What the timed step hands its caller after the last step -- the population (decision vectors, objectives, ranks)
+    and its hypervolume -- as ``out_dir/<name>.npy`` in float64.  Above ``limit_bytes`` a fixed, seeded sample of
+    population rows is written instead, with their indices in ``rows.npy``."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"population_x": rs.pop_x.download(), "population_y": rs.pop_y.download(), "rank": rs.rank.download().astype(np.float64)}
+    row_bytes = 8 * sum(a[0].size for a in arrays.values())  # written as float64
+    max_rows = max(1, (limit_bytes - 1024) // (row_bytes + 8))
+    if rs.pop > max_rows:
+        rows = np.sort(np.random.default_rng(seed).choice(rs.pop, size=max_rows, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    arrays["hypervolume"] = np.array([rs.hv], dtype=np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def time_device(L, fn, reps=3, warm=1):
     for _ in range(warm):
         fn()
@@ -529,6 +554,8 @@ def run_ours(args):
     prof = L.profile_report()
     L.profile_enable(False)
     clk = clocks.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, rs)
     value = n_val / t_val
     refined = sm._gp.auto_info()["last_refined"] if prec == L.GP_AUTO else 0
 
@@ -666,7 +693,11 @@ def main():
     ap.add_argument("--e2e-warmup", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sort-hv", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (population, ranks, hypervolume) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

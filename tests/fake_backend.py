@@ -1,7 +1,7 @@
 """Oracle-backed stand-in for ``dmosopt_b200._lib`` -- TEST SEAM ONLY.
 
 The product has no CPU path.  To exercise the *host* logic of the plugins (argument marshalling,
-state handling, dtype flow, the unmodified MOASMO.epoch driving them) in a container without a GPU,
+state handling, dtype flow) on a machine without a GPU,
 tests monkeypatch the thin ``_lib`` functions with these NumPy implementations built on ``oracle/``.
 """
 

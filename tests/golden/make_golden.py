@@ -3,7 +3,7 @@
 
 Run in the build container, where the reference checkout is mounted read-only:
 
-    PYTHONPATH=/root/reference PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
+    PYTHONPATH=<dmosopt checkout> PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py [name ...]
 
 It imports dmosopt's own modules (dda, indicators, MOEA, NSGA2, AGEMOEA, SMPSO,
 CMAES, hv, hv_box_decomposition, model + scikit-learn) and records seeded
@@ -277,7 +277,7 @@ def gen_gp(rng):
     from sklearn.gaussian_process import GaussianProcessRegressor
     from sklearn.gaussian_process.kernels import ConstantKernel, Matern, RBF, WhiteKernel
 
-    out = {}
+    out, factors = {}, {}
     k = 0
     cases = [
         # (N, d, M, P, kind, length_scale (None = fixed initial theta), anisotropic)
@@ -336,7 +336,7 @@ def gen_gp(rng):
         out[f"c{k}_var"] = var
         out[f"c{k}_Xtrain"] = np.asarray(smlist[0].X_train_)
         out[f"c{k}_alpha"] = np.stack([np.ravel(g.alpha_) for g in smlist])
-        out[f"c{k}_L"] = np.stack([g.L_ for g in smlist])
+        factors[f"c{k}_L"] = np.stack([g.L_ for g in smlist])
         out[f"c{k}_const"] = np.array([g.kernel_.k1.k1.constant_value for g in smlist])
         out[f"c{k}_ls"] = np.stack([np.broadcast_to(np.asarray(g.kernel_.k1.k2.length_scale, float), (d,)) for g in smlist])
         out[f"c{k}_noise"] = np.array([g.kernel_.k2.noise_level for g in smlist])
@@ -345,6 +345,7 @@ def gen_gp(rng):
         k += 1
     out["ncases"] = np.array(k)
     save("gp", **out)
+    save("gp_factors", **factors)  # the Cholesky factors in a file of their own: each file stays under 1 MB
 
 
 def gen_hv(rng):
@@ -798,8 +799,58 @@ def gen_trs(rng):
     save("trs", **out)
 
 
+def gen_reference_loop(rng):
+    """The reference's results for tests/test_gpu_reference_loop.py: three NSGA2 generations (its own generate / update) and
+    the controller helpers MOASMO.get_best, MOEA.get_duplicates / crowding_distance_metric and hv.AdaptiveHyperVolume."""
+    from dmosopt import MOASMO
+    from dmosopt import model as rmodel
+
+    out = {}
+    # ---- NSGA2: same initial state, the reference's offspring, the reference's survivors after each update
+    d, M, pop = 10, 3, 300
+    r = np.random.default_rng(3)
+    bounds = np.column_stack((np.zeros(d), np.ones(d)))
+    x0 = r.random((pop, d))
+
+    def f(x):
+        return np.column_stack((x[:, 0] + x[:, 3:].sum(1) * 0.1, (1 - x[:, 0]) * (1 + x[:, 1]), x[:, 2] ** 2 + 0.5 * x[:, 1]))
+
+    y0 = f(x0).astype(np.float32)
+    out["nsga2_x0"], out["nsga2_y0"] = x0, y0
+    ro = NSGA2.NSGA2(popsize=pop, nInput=d, nOutput=M, model=rmodel.Model(), distance_metric=None)
+    ro.initialize_strategy(x0.astype(np.float32), y0.copy(), bounds, np.random.default_rng(1))
+    out["nsga2_init_rank"] = np.array(ro.state.rank)  # copies: the reference updates its state arrays in place
+    for gi in range(3):
+        x_gen, st = ro.generate()
+        x_gen = np.array(x_gen)
+        ro.update(x_gen, f(x_gen), st)
+        out[f"nsga2_g{gi}_xgen"] = x_gen
+        out[f"nsga2_g{gi}_cidx"] = np.array(st["crossover_indices"])
+        out[f"nsga2_g{gi}_midx"] = np.array(st["mutation_indices"])
+        out[f"nsga2_g{gi}_rank"] = np.array(ro.state.rank)
+        out[f"nsga2_g{gi}_py"] = np.array(ro.state.population_obj)
+    # ---- controller helpers on a set with duplicated objective rows and shared decision rows
+    r = np.random.default_rng(21)
+    n, d, M = 700, 9, 3
+    x = r.random((n, d))
+    y = np.column_stack((x[:, 0] + 0.1, (1.1 - x[:, 0]) * (1 + x[:, 1]), 0.2 + x[:, 2] ** 2 + x[:, 1]))
+    y[50] = y[3]
+    y[400] = y[3]
+    x0 = r.random((300, d))
+    x0[:40] = x[100:140]
+    ref_pt = y.max(axis=0) + 0.1
+    out["help_x"], out["help_y"], out["help_x0"], out["help_ref"] = x, y, x0, ref_pt
+    best_x, best_y, best_f, best_c, best_epoch, perm = MOASMO.get_best(x, y, None, None, d, M, return_perm=True)
+    assert best_f is None and best_c is None and best_epoch is None
+    out["help_best_x"], out["help_best_y"], out["help_best_perm"] = best_x, best_y, np.asarray(perm)
+    out["help_dup"] = MOEA.get_duplicates(x, x0)
+    out["help_cd"] = MOEA.crowding_distance_metric(y[np.r_[0:50, 51:400, 401:n]])
+    out["help_hv"] = np.array(hv_mod.AdaptiveHyperVolume(ref_pt).compute_hypervolume(y[:300]))
+    save("reference_loop", **out)
+
+
 def main():
-    which = sys.argv[1:] or ["dda", "distance", "sortmo", "variation", "tournament", "duplicates", "gp", "hv", "ehvi", "nsga2", "agemoea", "smpso", "cmaes", "plugins", "trs", "adaptive", "hv_many"]
+    which = sys.argv[1:] or ["dda", "distance", "sortmo", "variation", "tournament", "duplicates", "gp", "hv", "ehvi", "nsga2", "agemoea", "smpso", "cmaes", "plugins", "trs", "adaptive", "hv_many", "reference_loop"]
     gens = {
         "dda": gen_dda,
         "distance": gen_distance,
@@ -818,6 +869,7 @@ def main():
         "trs": gen_trs,
         "adaptive": gen_adaptive,
         "hv_many": gen_hv_many,
+        "reference_loop": gen_reference_loop,
     }
     for i, name in enumerate(which):
         gens[name](np.random.default_rng(20260921 + i * 0 + sum(map(ord, name))))

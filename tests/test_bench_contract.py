@@ -2,11 +2,15 @@
 
 The GPU arm prints the same keys plus `roofline` (checked on the GPU box by the driver's own run); here the reference
 arm is run at a toy size so that the line's shape, the exact step count and the rank-0-only rule are covered.
+On the GPU arm, `--dump-outputs` is checked for identical outputs from two runs with the same arguments.
 """
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -51,3 +55,26 @@ def test_reference_arm_other_ranks_stay_silent():
     r = _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}, args=("--gpus", "2"))
     assert r.returncode == 0
     assert not [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_from_run_to_run(tmp_path):
+    """--dump-outputs: the last timed step's population, ranks and hypervolume as float64 .npy files, identical for two runs
+    with the same arguments; --steps is the number of timed steps."""
+    args = ["--steps", "3", "--warmup", "1", "--pop", "512", "--dim", "6", "--obj", "3", "--ntrain", "128", "--e2e-steps", "1",
+            "--no-cpu-baseline", "--no-sort-hv"]
+    dumps = []
+    for run in ("a", "b"):
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), *args, "--dump-outputs", str(tmp_path / run)]
+        r = subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][0])
+        assert d["steps"] == 3 and d["warmup"] == 1
+        dumps.append({f.stem: np.load(f) for f in sorted((tmp_path / run).iterdir())})
+    a, b = dumps
+    assert sorted(a) == ["hypervolume", "population_x", "population_y", "rank"]
+    assert a["population_x"].shape == (512, 6) and a["population_y"].shape == (512, 3) and a["rank"].shape == (512,)
+    assert all(v.dtype == np.float64 for v in a.values())
+    assert a["hypervolume"][0] == d["hypervolume"] > 0
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k

@@ -1,123 +1,49 @@
-"""The real thing on hardware: the UNMODIFIED reference controller loop (dmosopt/MOASMO.py:196-470, MOASMO.epoch) driving
-the B200 plugins by import path on the GPU, and the plain-C host of include/dmosopt_b200.h executed on the GPU.
+"""The reference's own results against the GPU plugins on hardware, and the plain-C host of include/dmosopt_b200.h executed
+on the GPU.
 
-The reference package is taken from ``baseline/_ref`` (the unmodified dmosopt modules installed there by pip from a copy
-of /root/reference, git-ignored, shipped to the GPU box by gpurun) or from ``$DMOSOPT_REF``; /root/reference itself is
-never read at run time.
+The reference's results come from tests/golden/reference_loop.npz (written by tests/golden/make_golden.py with dmosopt
+importable): three generations of its NSGA2 and its controller helpers (MOASMO.get_best, MOEA.get_duplicates /
+crowding_distance_metric, hv.AdaptiveHyperVolume) on seeded inputs.
 """
 
 import os
 import shutil
 import subprocess
 import sys
+import types
 
 import numpy as np
 import pytest
+
+from conftest import load_golden
 
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _reference_path():
-    for p in (os.environ.get("DMOSOPT_REF"), os.path.join(ROOT, "baseline", "_ref")):
-        if p and os.path.isdir(os.path.join(p, "dmosopt")):
-            return p
-    return None
-
-
-def _zdt1(x):
-    d = x.shape[1]
-    g = 1.0 + 9.0 / (d - 1) * x[:, 1:].sum(axis=1)
-    return np.column_stack((x[:, 0], g * (1.0 - np.sqrt(x[:, 0] / g))))
-
-
-@pytest.mark.skipif(_reference_path() is None, reason="reference package not shipped (baseline/_ref or $DMOSOPT_REF)")
-@pytest.mark.parametrize("optimizer,kwargs", [("dmosopt_b200.NSGA2", {}), ("dmosopt_b200.AGEMOEA", {}), ("dmosopt_b200.SMPSO", {}), ("dmosopt_b200.CMAES", {})])
-def test_unmodified_moasmo_epoch_drives_the_gpu_plugins(optimizer, kwargs):
-    """MOASMO.epoch resolves optimizer_name / surrogate_method_name by import path (config.py:5-11), fits the surrogate
-    (GPR_Matern, default precision = auto), runs the generation loop on the GPU and the resample step
-    (MOEA.get_duplicates(best_x, x_0) + crowding, MOASMO.py:441-448)."""
-    ref = _reference_path()
-    sys.path.insert(0, ref)
-    try:
-        from dmosopt import MOASMO
-    finally:
-        sys.path.remove(ref)
-    from dmosopt_b200 import _lib
-
-    _lib.context()
-    d, M, pop = 8, 2, 64
-    rng = np.random.default_rng(11)
-    xlb, xub = np.zeros(d), np.ones(d)
-    X = rng.random((120, d))
-    Y = _zdt1(X)
-    launches0 = _lib.launch_count()
-    gen = MOASMO.epoch(
-        6, [f"x{i}" for i in range(d)], ["y1", "y2"], xlb, xub, 0.25, X, Y, None, pop=pop,
-        optimizer_name=optimizer, optimizer_kwargs=kwargs, surrogate_method_name="dmosopt_b200.GPR_Matern",
-        surrogate_method_kwargs={"anisotropic": False, "optimizer": None}, local_random=rng,
-    )
-    try:
-        next(gen)
-        raise AssertionError("epoch should finish without yielding when a surrogate is present")
-    except StopIteration as ex:
-        res = ex.args[0]
-    assert _lib.launch_count() > launches0  # the generations ran on the GPU library
-    assert type(res["optimizer"]).__module__.startswith("dmosopt_b200")
-    xr, yp = res["x_resample"], res["y_pred"]
-    assert xr.shape[1] == d and len(xr) > 0 and yp.shape == (len(xr), M)
-    assert np.all(xr >= xlb) and np.all(xr <= xub)
-    # the resampled points are predicted to improve on the training set: their predicted objectives are not dominated
-    # by the bulk of the initial sample (ZDT1: f2 falls as the surrogate pushes g towards 1)
-    assert np.median(yp[:, 1]) < np.median(Y[:, 1])
-    # predictions stored by the epoch agree with the oracle restatement of the fitted model at the resampled points
-    from oracle import gp as ogp
-
-    sm = res["optimizer"].model.objective if hasattr(res["optimizer"], "model") else None
-    if sm is not None and hasattr(sm, "smlist"):
-        st = ogp.from_sklearn(sm.smlist, xlb, xub)
-        mean_o, _ = ogp.predict(st, xr)
-        ystd = np.array([o.y_std for o in st.objectives])
-        assert np.max(np.abs(mean_o - yp) / np.maximum(np.abs(mean_o), ystd)) < 1e-5
-
-
-@pytest.mark.skipif(_reference_path() is None, reason="reference package not shipped")
 def test_reference_and_plugin_nsga2_agree_on_a_generation():
     """Same initial state and the same offspring: the reference's NSGA2.update_strategy (dda_ens + sortMO on the CPU)
     and the GPU plugin keep the same survivors, in the same order, with the same ranks."""
-    ref = _reference_path()
-    sys.path.insert(0, ref)
-    try:
-        from dmosopt import NSGA2 as rNSGA2
-        from dmosopt import model as rmodel
-    finally:
-        sys.path.remove(ref)
     import dmosopt_b200 as b2
 
-    d, M, pop = 10, 3, 300
-    rng = np.random.default_rng(3)
+    g = load_golden("reference_loop")
+    x0, y0 = g["nsga2_x0"], g["nsga2_y0"]
+    pop, d = x0.shape
+    M = y0.shape[1]
     bounds = np.column_stack((np.zeros(d), np.ones(d)))
-    x0 = rng.random((pop, d))
 
     def f(x):
         return np.column_stack((x[:, 0] + x[:, 3:].sum(1) * 0.1, (1 - x[:, 0]) * (1 + x[:, 1]), x[:, 2] ** 2 + 0.5 * x[:, 1]))
 
-    y0 = f(x0).astype(np.float32)
-    ro = rNSGA2.NSGA2(popsize=pop, nInput=d, nOutput=M, model=rmodel.Model(), distance_metric=None)
-    ro.initialize_strategy(x0.astype(np.float32), y0.copy(), bounds, np.random.default_rng(1))
     bo = b2.NSGA2(popsize=pop, nInput=d, nOutput=M, model=None, distance_metric=None)
     bo.initialize_strategy(x0.astype(np.float32), y0.copy(), bounds, np.random.default_rng(1))
-    assert np.array_equal(ro.state.rank, bo.state.rank)
-    for _ in range(3):
-        x_gen, st = bo.generate()
-        x_gen = np.array(x_gen)
-        y_gen = f(x_gen)
-        ro.state.population_parm = np.array(bo.state.population_parm, dtype=np.float32) if ro.state.population_parm.dtype == np.float32 else np.array(bo.state.population_parm)
-        ro.update(x_gen, y_gen, {"crossover_indices": st["crossover_indices"], "mutation_indices": st["mutation_indices"]})
-        bo.update(x_gen, y_gen, st)
-        assert np.array_equal(np.asarray(ro.state.rank), np.asarray(bo.state.rank))
-        assert np.array_equal(np.asarray(ro.state.population_obj), np.asarray(bo.state.population_obj))
+    assert np.array_equal(g["nsga2_init_rank"], bo.state.rank)
+    for gi in range(3):
+        x_gen = g[f"nsga2_g{gi}_xgen"]  # the reference's own offspring of this generation
+        bo.update(x_gen, f(x_gen), {"crossover_indices": g[f"nsga2_g{gi}_cidx"], "mutation_indices": g[f"nsga2_g{gi}_midx"]})
+        assert np.array_equal(g[f"nsga2_g{gi}_rank"], np.asarray(bo.state.rank)), gi
+        assert np.array_equal(g[f"nsga2_g{gi}_py"], np.asarray(bo.state.population_obj)), gi
 
 
 def test_plain_c_host_runs_the_resident_step_on_the_gpu(tmp_path):
@@ -138,51 +64,66 @@ def test_plain_c_host_runs_the_resident_step_on_the_gpu(tmp_path):
     assert all(b >= a - 1e-12 for a, b in zip(hv, hv[1:])), hv  # elitist survival: the hypervolume never shrinks
 
 
-@pytest.mark.skipif(_reference_path() is None, reason="reference package not shipped")
-def test_install_routes_controller_helpers_to_the_gpu_with_identical_results():
+def _standin_package(monkeypatch, name):
+    """A package shaped like dmosopt's MOEA / indicators / dda / hv modules whose helpers fail when called: whatever
+    answers after install() was routed to the GPU library."""
+
+    def unrouted(*args, **kwargs):
+        raise AssertionError("stand-in helper called: install() did not route it")
+
+    class AdaptiveHyperVolume:
+        def __init__(self, ref_point, dimension_threshold_exact=10):
+            self.ref_point = np.asarray(ref_point, dtype=np.float64)
+            self.n_objectives = len(ref_point)
+            self.dimension_threshold_exact = dimension_threshold_exact
+
+        compute_hypervolume = unrouted
+
+    mods = {}
+    for sub, attrs in (("MOEA", ("get_duplicates", "remove_duplicates", "sortMO", "orderMO", "remove_worst", "crowding_distance_metric", "dda_ens")),
+                       ("indicators", ("crowding_distance_metric", "euclidean_distance_metric")), ("dda", ("dda_ens",)), ("hv", ())):
+        m = types.ModuleType(f"{name}.{sub}")
+        for a in attrs:
+            setattr(m, a, unrouted)
+        mods[sub] = m
+    mods["hv"].AdaptiveHyperVolume = AdaptiveHyperVolume
+    monkeypatch.setitem(sys.modules, name, types.ModuleType(name))
+    for sub, m in mods.items():
+        monkeypatch.setitem(sys.modules, f"{name}.{sub}", m)
+    return mods
+
+
+def test_install_routes_controller_helpers_to_the_gpu_with_identical_results(monkeypatch):
     """dmosopt_b200.install(): MOASMO.get_best (duplicates + sortMO, MOASMO.py:581-639), the resample helpers
-    (MOASMO.py:441-448) and the termination hypervolume (hv.py:123-189) give the reference's own results -- computed
-    first with the untouched reference, then again after the routing hook."""
-    ref = _reference_path()
-    sys.path.insert(0, ref)
-    try:
-        import dmosopt.hv as rhv
-        import dmosopt.MOASMO as rMOASMO
-        import dmosopt.MOEA as rMOEA
-    finally:
-        sys.path.remove(ref)
+    (MOASMO.py:441-448) and the termination hypervolume (hv.py:123-189) give the reference's own results once routed
+    to the GPU, and uninstall() restores the module attributes."""
     import dmosopt_b200 as b2
     from dmosopt_b200 import _lib
 
-    rng = np.random.default_rng(21)
-    n, d, M = 700, 9, 3
-    x = rng.random((n, d))
-    y = np.column_stack((x[:, 0] + 0.1, (1.1 - x[:, 0]) * (1 + x[:, 1]), 0.2 + x[:, 2] ** 2 + x[:, 1]))
-    y[50] = y[3]
-    y[400] = y[3]
-    x0 = rng.random((300, d))
-    x0[:40] = x[100:140]
-    ref_pt = y.max(axis=0) + 0.1
-    # reference results, untouched
-    best_ref = rMOASMO.get_best(x, y, None, None, d, M, return_perm=True)
-    dup_ref = rMOEA.get_duplicates(x, x0)
-    y_tf = y[np.r_[0:50, 51:400, 401:n]]  # tie-free columns: with exact ties the reference's own crowding depends on argsort's order
-    cd_ref = rMOEA.crowding_distance_metric(y_tf)
-    hv_ref = rhv.AdaptiveHyperVolume(ref_pt).compute_hypervolume(y[:300])
+    g = load_golden("reference_loop")
+    x, y, x0, ref_pt = g["help_x"], g["help_y"], g["help_x0"], g["help_ref"]
+    n = x.shape[0]
+    mods = _standin_package(monkeypatch, "dmosopt_standin")
+    rMOEA, rhv = mods["MOEA"], mods["hv"]
+    originals = {a: getattr(rMOEA, a) for a in ("get_duplicates", "sortMO", "crowding_distance_metric", "dda_ens")}
     launches0 = _lib.launch_count()
-    patched = b2.install()
+    patched = b2.install("dmosopt_standin")
     try:
         assert any(name.endswith("get_duplicates") for name in patched)
-        best_gpu = rMOASMO.get_best(x, y, None, None, d, M, return_perm=True)
+        # MOASMO.get_best without constraints or epochs: duplicates of y dropped, then the rank-0 rows of sortMO's order
+        dup_y = rMOEA.get_duplicates(y)
+        xs, ys, rank, _, perm = rMOEA.sortMO(x[~dup_y], y[~dup_y], return_perm=True)
         dup_gpu = rMOEA.get_duplicates(x, x0)
+        y_tf = y[np.r_[0:50, 51:400, 401:n]]  # tie-free columns: with exact ties the reference's own crowding depends on argsort's order
         cd_gpu = rMOEA.crowding_distance_metric(y_tf)
         hv_gpu = rhv.AdaptiveHyperVolume(ref_pt).compute_hypervolume(y[:300])
     finally:
         b2.uninstall()
     assert _lib.launch_count() > launches0
-    assert rMOEA.get_duplicates.__module__.startswith("dmosopt.")  # restored
-    for a, b in zip(best_ref, best_gpu):
-        assert (a is None and b is None) or np.array_equal(np.asarray(a), np.asarray(b))
-    assert np.array_equal(dup_ref, dup_gpu) and dup_ref.sum() == 40
-    assert np.array_equal(cd_ref, cd_gpu)  # float64 bit-exact crowding (tie-free columns)
+    assert all(getattr(rMOEA, a) is fn for a, fn in originals.items())  # restored
+    assert np.array_equal(xs[rank == 0], g["help_best_x"]) and np.array_equal(ys[rank == 0], g["help_best_y"])
+    assert np.array_equal(np.asarray(perm), g["help_best_perm"])
+    assert np.array_equal(g["help_dup"], dup_gpu) and g["help_dup"].sum() == 40
+    assert np.array_equal(g["help_cd"], cd_gpu)  # float64 bit-exact crowding (tie-free columns)
+    hv_ref = float(g["help_hv"])
     assert abs(hv_gpu - hv_ref) <= 1e-9 * abs(hv_ref)
