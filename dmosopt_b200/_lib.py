@@ -729,7 +729,9 @@ class GPHandle:
         em, ev, th = _c_dbl(0.0), _c_dbl(0.0), _c_dbl(0.0)
         _check(load_library().dmo_gp_auto_info(context(), self._h, ctypes.byref(mt), ctypes.byref(vt), ctypes.byref(em), ctypes.byref(ev),
                                                ctypes.byref(th), ctypes.byref(rows)), "dmo_gp_auto_info")
-        return {"mean_tensor": bool(mt.value & 3), "mean_from_contraction": bool(mt.value & 2), "mean_only_tensor": bool(mt.value & 4),
+        # mean_from_contraction is always False (bit 1 is reserved); the key stays so that the dict, which bench.py
+        # records as gp_auto, keeps its shape
+        return {"mean_tensor": bool(mt.value & 1), "mean_from_contraction": bool(mt.value & 2), "mean_only_tensor": bool(mt.value & 4),
                 "var_tensor": bool(vt.value), "mean_err": em.value,
                 "var_err": ev.value, "theta": th.value, "last_refined": int(rows.value)}
 

@@ -16,10 +16,8 @@
 struct dmo_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
-  cudaStream_t aux = nullptr;  // second stream: producer kernels that overlap a consumer on `stream` (gp_tensor.cu)
   cudaMemPool_t pool = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;  // stream <-> aux ordering
   int sm_count = 148;
   int64_t launches = 0;
   std::string err;
@@ -40,18 +38,17 @@ struct dmo_ctx {
 struct ProfileScope {
   dmo_ctx* ctx;
   int idx = -1;
-  cudaStream_t st;
-  ProfileScope(dmo_ctx* c, const char* name, cudaStream_t on = nullptr) : ctx(c), st(on ? on : c->stream) {
+  ProfileScope(dmo_ctx* c, const char* name) : ctx(c) {
     if (!c->profiling) return;
     dmo_ctx::Timer t;
     t.name = name;
     if (cudaEventCreate(&t.a) != cudaSuccess || cudaEventCreate(&t.b) != cudaSuccess) return;
-    cudaEventRecord(t.a, st);
+    cudaEventRecord(t.a, c->stream);
     c->timers.push_back(t);
     idx = (int)c->timers.size() - 1;
   }
   ~ProfileScope() {
-    if (idx >= 0) cudaEventRecord(ctx->timers[idx].b, st);
+    if (idx >= 0) cudaEventRecord(ctx->timers[idx].b, ctx->stream);
   }
 };
 
@@ -81,13 +78,6 @@ int dmo_fail(dmo_ctx* ctx, int code, const char* fmt, ...);
 #define DMO_LAUNCH(kernel, grid, block, smem, ...)                       \
   do {                                                                   \
     kernel<<<(grid), (block), (smem), ctx->stream>>>(__VA_ARGS__);       \
-    ctx->launches++;                                                     \
-  } while (0)
-
-// the same on an explicit stream (the context's aux stream)
-#define DMO_LAUNCH_ON(strm, kernel, grid, block, smem, ...)              \
-  do {                                                                   \
-    kernel<<<(grid), (block), (smem), (strm)>>>(__VA_ARGS__);            \
     ctx->launches++;                                                     \
   } while (0)
 

@@ -47,10 +47,7 @@ int dmo_create(int device, dmo_ctx** out) {
   }
   ctx->sm_count = prop.multiProcessorCount;
   if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaStreamCreateWithFlags(&ctx->aux, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaEventCreate(&ctx->ev0) != cudaSuccess || cudaEventCreate(&ctx->ev1) != cudaSuccess ||
-      cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming) != cudaSuccess) {
+      cudaEventCreate(&ctx->ev0) != cudaSuccess || cudaEventCreate(&ctx->ev1) != cudaSuccess) {
     delete ctx;
     return DMO_ERR_CUDA;
   }
@@ -74,12 +71,8 @@ int dmo_destroy(dmo_ctx* ctx) {
   cudaStreamSynchronize(ctx->stream);
   if (ctx->flush_buf) cudaFree(ctx->flush_buf);
   if (ctx->dev_flag) cudaFree(ctx->dev_flag);
-  cudaStreamSynchronize(ctx->aux);
   cudaEventDestroy(ctx->ev0);
   cudaEventDestroy(ctx->ev1);
-  cudaEventDestroy(ctx->ev_fork);
-  cudaEventDestroy(ctx->ev_join);
-  cudaStreamDestroy(ctx->aux);
   cudaStreamDestroy(ctx->stream);
   delete ctx;
   return DMO_OK;

@@ -105,17 +105,6 @@ __global__ void copy_pad_kernel(const double* __restrict__ src, int64_t rows, in
   dst[r * ldo + c] = src[t];
 }
 
-// z[i] = sum_{r >= i} L[r][i] alpha[r]  (= L' alpha = L^-1 y_n), float, zero tail up to Npad
-__global__ void whitened_targets_kernel(const double* __restrict__ L, int64_t N, const double* __restrict__ alpha, int64_t Npad,
-                                        float* __restrict__ z) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= Npad) return;
-  double s = 0.0;
-  if (i < N)
-    for (int64_t r = i; r < N; ++r) s += L[r * N + i] * alpha[r];
-  z[i] = (float)s;
-}
-
 __global__ void normalise_x_kernel(const double* __restrict__ X, int64_t P, int d, const double* __restrict__ xlb,
                                    const double* __restrict__ xrg, double* __restrict__ Xn) {
   int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -476,18 +465,14 @@ int gp_calibrate(dmo_ctx* ctx, dmo_gp* gp) {
   DMO_CHECK_LAUNCH();
   const bool prof = ctx->profiling;
   ctx->profiling = false;  // calibration launches are not part of any timed step
-  DevBuf<double> md, mo;
-  DMO_TRY(md.alloc(ctx, (size_t)P * M));
+  DevBuf<double> mo;
   DMO_TRY(mo.alloc(ctx, (size_t)P * M));
   int rc = gp_predict_fp64(ctx, gp, xn.p, P, m64.p, v64.p);
-  if (rc == DMO_OK) rc = gp_predict_tensor(ctx, gp, xn.p, P, mt.p, vt.p, false);
-  if (rc == DMO_OK) rc = gp_predict_tensor(ctx, gp, xn.p, P, mo.p, nullptr, false);  // the mean-only call takes its own kernel
-  const bool try_d = gp->z_ready;
-  if (rc == DMO_OK && try_d) rc = gp_predict_tensor(ctx, gp, xn.p, P, md.p, vt.p, true);  // same variance, mean from D z
+  if (rc == DMO_OK) rc = gp_predict_tensor(ctx, gp, xn.p, P, mt.p, vt.p);
+  if (rc == DMO_OK) rc = gp_predict_tensor(ctx, gp, xn.p, P, mo.p, nullptr);  // the mean-only call takes its own kernel
   ctx->profiling = prof;
   if (rc != DMO_OK) return rc;
-  std::vector<double> h((size_t)4 * P * M), hd((size_t)P * M), ho((size_t)P * M);
-  if (try_d) DMO_CUDA(cudaMemcpyAsync(hd.data(), md.p, (size_t)P * M * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  std::vector<double> h((size_t)4 * P * M), ho((size_t)P * M);
   DMO_CUDA(cudaMemcpyAsync(ho.data(), mo.p, (size_t)P * M * 8, cudaMemcpyDeviceToHost, ctx->stream));
   DMO_CUDA(cudaMemcpyAsync(h.data(), m64.p, (size_t)P * M * 8, cudaMemcpyDeviceToHost, ctx->stream));
   DMO_CUDA(cudaMemcpyAsync(h.data() + (size_t)P * M, v64.p, (size_t)P * M * 8, cudaMemcpyDeviceToHost, ctx->stream));
@@ -495,7 +480,7 @@ int gp_calibrate(dmo_ctx* ctx, dmo_gp* gp) {
   DMO_CUDA(cudaMemcpyAsync(h.data() + (size_t)3 * P * M, vt.p, (size_t)P * M * 8, cudaMemcpyDeviceToHost, ctx->stream));
   DMO_CUDA(cudaStreamSynchronize(ctx->stream));
   const double *a64 = h.data(), *b64 = a64 + (size_t)P * M, *at = b64 + (size_t)P * M, *bt = at + (size_t)P * M;
-  double em = 0.0, ev = 0.0, ed = try_d ? 0.0 : INFINITY, eo = 0.0;
+  double em = 0.0, ev = 0.0, eo = 0.0;
   for (int p = 0; p < P; ++p)
     for (int m = 0; m < M; ++m) {
       const double ys = gp->h_ystd[m];
@@ -504,27 +489,20 @@ int gp_calibrate(dmo_ctx* ctx, dmo_gp* gp) {
       const double dv = fabs(bt[p * M + m] - b64[p * M + m]) / prior;
       em = (dm > em || dm != dm) ? (dm != dm ? INFINITY : dm) : em;
       ev = (dv > ev || dv != dv) ? (dv != dv ? INFINITY : dv) : ev;
-      if (try_d) {
-        const double dd = fabs(hd[p * M + m] - a64[p * M + m]) / fmax(fabs(a64[p * M + m]), ys);
-        ed = (dd > ed || dd != dd) ? (dd != dd ? INFINITY : dd) : ed;
-      }
       const double dq = fabs(ho[p * M + m] - a64[p * M + m]) / fmax(fabs(a64[p * M + m]), ys);
       eo = (dq > eo || dq != dq) ? (dq != dq ? INFINITY : dq) : eo;
     }
   gp->cal_mean_err = em;
-  gp->cal_mean_err_d = ed;
   gp->cal_mean_err_only = eo;
   gp->cal_var_err = ev;
-  // the mean out of the contraction saves the K_* alpha pass; it is used when it holds the same margin on the probes
-  gp->mean_from_d = try_d && ed <= 2.5e-6;
   gp->auto_mean_tensor = em <= 2.5e-6;
   gp->auto_mean_only = eo <= 2.5e-6;
-  gp->auto_var_tensor = (gp->auto_mean_tensor || gp->mean_from_d) && ev <= 4.5e-6;
+  gp->auto_var_tensor = gp->auto_mean_tensor && ev <= 4.5e-6;
   gp->refine_theta = fmax(0.02, 2.0 * ev / 1e-5);
   gp->calibrated = true;
   if (getenv("DMO_GP_VERBOSE"))
-    fprintf(stderr, "dmosopt_b200: GP calibration (N=%lld d=%d M=%d): mean err K*alpha %.3e, D z %.3e, mean-only kernel %.3e, var err/prior %.3e -> mean %s, var %s, theta %.3f\n",
-            (long long)gp->N, d, M, em, ed, eo, ev, gp->mean_from_d ? "contraction" : (gp->auto_mean_tensor ? "K*alpha pass" : "float64"),
+    fprintf(stderr, "dmosopt_b200: GP calibration (N=%lld d=%d M=%d): mean err K*alpha %.3e, mean-only kernel %.3e, var err/prior %.3e -> mean %s, var %s, theta %.3f\n",
+            (long long)gp->N, d, M, em, eo, ev, gp->auto_mean_tensor ? "K*alpha pass" : "float64",
             gp->auto_var_tensor ? "tensor" : "float64", gp->refine_theta);
   return DMO_OK;
 }
@@ -537,7 +515,7 @@ int gp_predict_auto(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, doub
     gp->last_refined = P;
     return gp_predict_fp64(ctx, gp, dXn, P, d_mean, d_var);
   }
-  DMO_TRY(gp_predict_tensor(ctx, gp, dXn, P, d_mean, d_var, d_var != nullptr && gp->mean_from_d));
+  DMO_TRY(gp_predict_tensor(ctx, gp, dXn, P, d_mean, d_var));
   if (!d_var) return DMO_OK;
   const int M = gp->M, d = gp->d;
   DevBuf<int32_t> flag, pos;
@@ -651,14 +629,6 @@ int dmo_gp_create(dmo_ctx* ctx, int64_t N, int d, int M, int kernel, const doubl
       if (factor_is_inverse) {
         DMO_LAUNCH(copy_pad_kernel, (unsigned)ceil_div(N * N, 256), 256, 0, src, N, N, Npad, dst);
       } else {
-        // experimental (DMO_GP_MEAN_D=1): whitened targets for taking the mean out of the variance contraction (D z).  Off by
-        // default: on the BASELINE model its probe error is 7.9e-6 (the K_* alpha pass: 2.9e-7), outside the 2.5e-6 margin
-        if (getenv("DMO_GP_MEAN_D") && atoi(getenv("DMO_GP_MEAN_D"))) {
-          if (m == 0) GP_TRY(gp->Zf.alloc(ctx, (size_t)M * Npad));
-          DMO_LAUNCH(whitened_targets_kernel, (unsigned)ceil_div(Npad, 128), 128, 0, src, N, gp->alpha.p + (size_t)m * N, Npad,
-                     gp->Zf.p + (size_t)m * Npad);
-          gp->z_ready = true;
-        }
         int64_t Np = TRI_B;
         while (Np < N) Np *= 2;
         DevBuf<double> Lp, X, T;
@@ -749,9 +719,9 @@ int dmo_gp_auto_info(dmo_ctx* ctx, dmo_gp* gp, int* mean_tensor, int* var_tensor
   DMO_CUDA(cudaSetDevice(ctx->device));
   DMO_REQUIRE(gp, "gp_auto_info: null model");
   DMO_TRY(gp_calibrate(ctx, gp));
-  if (mean_tensor) *mean_tensor = (gp->auto_mean_tensor ? 1 : 0) | (gp->mean_from_d ? 2 : 0) | (gp->auto_mean_only ? 4 : 0);
+  if (mean_tensor) *mean_tensor = (gp->auto_mean_tensor ? 1 : 0) | (gp->auto_mean_only ? 4 : 0);
   if (var_tensor) *var_tensor = gp->auto_var_tensor ? 1 : 0;
-  if (mean_err) *mean_err = gp->mean_from_d ? fmax(gp->cal_mean_err_d, gp->auto_mean_tensor ? gp->cal_mean_err : 0.0) : gp->cal_mean_err;
+  if (mean_err) *mean_err = gp->cal_mean_err;
   if (var_err) *var_err = gp->cal_var_err;
   if (theta) *theta = gp->refine_theta;
   if (last_refined) *last_refined = gp->last_refined;

@@ -25,15 +25,9 @@ struct dmo_gp {
   DevBuf<int> Kexp;           // (M,) K_* scaling exponents
   DevBuf<float> Xtf;          // (Npad, 32) float copy of Xt, zero padded (mean-only direct kernel, d <= 32); built lazily
   DevBuf<float> CAf;          // (M, Npad) c_m * alpha_m as float, zero padded (fused K_* + mean kernel); built with Xtf
-  // whitened targets z = L^-1 y_n = L' alpha (float), zero padded to Npad: with D = K_* L^-T the posterior mean is D z, so
-  // the variance contraction's epilogue delivers it from the accumulator it already reads (gp_tensor.cu)
-  DevBuf<float> Zf;           // (M, Npad); empty when the model was created from L^-1 (factor_is_inverse)
-  bool z_ready = false;
-  bool mean_from_d = false;   // chosen by the AUTO calibration: mean from the contraction instead of the K_* alpha pass
   // DMO_GP_AUTO: per-model calibration of the tensor path against the float64 path on probe candidates (gp.cu)
   bool calibrated = false;
-  bool auto_mean_tensor = false;  // a tensor-path mean (K_* alpha pass or D z) holds 1e-5 on the probes (with margin)
-  double cal_mean_err_d = 0.0;    // probe error of the mean taken from the contraction (D z)
+  bool auto_mean_tensor = false;  // the tensor-path mean of predicts with variance holds 1e-5 on the probes (with margin)
   bool auto_var_tensor = false;   // split-fp16 variance holds 1e-5 * prior on the probes (with margin)
   double cal_mean_err = 0.0;      // max |mean_t - mean_64| / max(|mean_64|, y_std) over the probes
   bool auto_mean_only = false;    // the mean-only tensor-path call (direct kernel where it applies) holds 1e-5 on the probes
@@ -44,5 +38,4 @@ struct dmo_gp {
 };
 
 int gp_predict_fp64(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, double* d_mean, double* d_var);
-// mean_from_d: take the mean from the variance contraction (needs d_var and gp->z_ready), else from the K_* alpha pass
-int gp_predict_tensor(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, double* d_mean, double* d_var, bool mean_from_d = false);
+int gp_predict_tensor(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, double* d_mean, double* d_var);

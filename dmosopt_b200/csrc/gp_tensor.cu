@@ -13,7 +13,7 @@
 //   * operand tiles arrive by TMA (cp.async.bulk.tensor, SWIZZLE_64B) into a 3-stage shared-memory ring, completion
 //     on mbarriers; one elected thread issues the MMAs; tcgen05.commit releases the ring slots and publishes the
 //     accumulator; four epilogue warps drain TMEM with tcgen05.ld;
-//   * persistent CTAs (one per SM) walk a list of equal-cost work items in an L2-friendly order (version 3, below).
+//   * persistent CTAs (one per SM) walk a list of equal-cost work items in an L2-friendly order (gp_var_tc3_kernel).
 //
 // K_* itself is produced in fp32 (relative error ~1e-6 on K_*) by kstar_mean_kernel, which accumulates the mean from the same
 // kernel values (packed fp32 over 16 training points, then float64, slices added in a fixed order: deterministic);
@@ -26,7 +26,6 @@
 #include <cuda.h>
 #include <cuda_fp16.h>
 #include <cudaTypedefs.h>
-#include <stdlib.h>
 
 #include "gp.cuh"
 
@@ -121,217 +120,34 @@ __device__ __forceinline__ void tc_ld_32x32(uint32_t taddr, uint32_t (&r)[32]) {
 }
 __device__ __forceinline__ void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
-// K-major, SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor, mma_sm100_desc.hpp):
-//   [0,14) start address >> 4 | [16,30) leading byte offset >> 4 (unused for swizzled K-major: 1)
-//   [32,46) stride byte offset >> 4 (8 rows x 128 B = 1024 B between 8-row groups) | [46,48) version = 1
-//   [61,64) layout type = 2 (SWIZZLE_128B)
-__device__ __forceinline__ uint64_t make_sdesc(uint32_t smem_addr) {
-  return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | (1ull << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) |
-         (2ull << 61);
-}
-
 // kind::f16 instruction descriptor (cute::UMMA::InstrDescriptor): fp16 A/B (format 0), fp32 accumulate (c_format 1),
 // both K-major, N >> 3 at [17,23), M >> 4 at [24,29)
 constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(TN >> 3) << 17) | ((uint32_t)(TM >> 4) << 24);
 
-// ------------------------------------------------------------------------------------------------ the GEMM, version 2
-// Same contraction, 1.5x less L2 -> shared-memory traffic per MMA: a work item owns 256 candidates (two M = 128
-// sub-tiles that share every Linv tile), k is staged 32 elements at a time (64-byte rows, SWIZZLE_64B) so that three
-// 64 KiB stages fit, both TMEM accumulators (2 x 256 columns) belong to the two sub-tiles, and the Linv row blocks of a
-// candidate block are split into two halves of equal MMA count (two work items, partial sums added in a fixed order)
-// to keep the tail of the persistent schedule short.
-namespace v2 {
-constexpr int TM2 = 256, TN2 = 256, TK2 = 32, STAGES2 = 3;
-constexpr int TILE_BYTES2 = 256 * TK2 * 2;             // 16 KiB: 256 rows x 64 B
-constexpr int STAGE_BYTES2 = 4 * TILE_BYTES2;          // K* hi/lo + Linv hi/lo
-constexpr size_t GEMM_SMEM2 = (size_t)STAGES2 * STAGE_BYTES2 + 1024 + 256;
-
-// K-major SWIZZLE_64B descriptor: 8-row groups are 512 B apart, layout type 4
-__device__ __forceinline__ uint64_t make_sdesc64(uint32_t smem_addr) {
-  return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | (1ull << 16) | ((uint64_t)(512 >> 4) << 32) | (1ull << 46) | (4ull << 61);
-}
-
-struct GemmParams2 {
-  int M, n_pb, n_jt, j_split;  // row blocks [0, j_split) belong to half 0, [j_split, n_jt) to half 1
-  int64_t k_rows, l_rows;
-  const float* inv_scale;
-  double* vnorm;  // [2][M][vn_ld]
-  int64_t vn_ld;
-  int* abort_flag;
-};
-
-__global__ void __launch_bounds__(NTHREADS, 1)
-    gp_var_tc2_kernel(const __grid_constant__ CUtensorMap map_kh, const __grid_constant__ CUtensorMap map_kl,
-                      const __grid_constant__ CUtensorMap map_lh, const __grid_constant__ CUtensorMap map_ll,
-                      const GemmParams2 prm) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* tiles = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  uint64_t* bars = (uint64_t*)(tiles + (size_t)STAGES2 * STAGE_BYTES2);
-  uint64_t* full = bars;
-  uint64_t* empty = bars + STAGES2;
-  uint64_t* acc_full = bars + 2 * STAGES2;
-  uint64_t* acc_empty = bars + 2 * STAGES2 + 1;
-  uint32_t* tmem_slot = (uint32_t*)(bars + 2 * STAGES2 + 2);
-  volatile int* abort_flag = prm.abort_flag;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < STAGES2; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], 1);
-    }
-    mbar_init(acc_full, 1);
-    mbar_init(acc_empty, 4);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 2) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const int n_work = prm.M * prm.n_pb * 2;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      uint32_t stage = 0, phase = 0;
-      for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
-        const int z = w & 1, wp = w >> 1;
-        const int m = wp / prm.n_pb, pb = wp - m * prm.n_pb;
-        const int a_row = (int)(m * prm.k_rows + (int64_t)pb * TM2);
-        const int j0 = z ? prm.j_split : 0, j1 = z ? prm.n_jt : prm.j_split;
-        for (int jt = j0; jt < j1; ++jt) {
-          const int b_row = (int)(m * prm.l_rows + (int64_t)jt * TN2);
-          const int nkc = (jt + 1) * (TN2 / TK2);
-          for (int kc = 0; kc < nkc; ++kc) {
-            mbar_wait(&empty[stage], phase ^ 1u, abort_flag);
-            uint8_t* st = tiles + (size_t)stage * STAGE_BYTES2;
-            mbar_expect_tx(&full[stage], STAGE_BYTES2);
-            tma_load_2d(&map_kh, &full[stage], st, kc * TK2, a_row);
-            tma_load_2d(&map_kl, &full[stage], st + TILE_BYTES2, kc * TK2, a_row);
-            tma_load_2d(&map_lh, &full[stage], st + 2 * TILE_BYTES2, kc * TK2, b_row);
-            tma_load_2d(&map_ll, &full[stage], st + 3 * TILE_BYTES2, kc * TK2, b_row);
-            if (++stage == STAGES2) {
-              stage = 0;
-              phase ^= 1u;
-            }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      uint32_t stage = 0, phase = 0, acc_phase = 0;
-      for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
-        const int z = w & 1;
-        const int j0 = z ? prm.j_split : 0, j1 = z ? prm.n_jt : prm.j_split;
-        for (int jt = j0; jt < j1; ++jt) {
-          mbar_wait(acc_empty, acc_phase ^ 1u, abort_flag);
-          tc_fence_after();
-          const int nkc = (jt + 1) * (TN2 / TK2);
-          for (int kc = 0; kc < nkc; ++kc) {
-            mbar_wait(&full[stage], phase, abort_flag);
-            tc_fence_after();
-            const uint32_t sa = smem_u32(tiles + (size_t)stage * STAGE_BYTES2);
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-              const uint32_t d_tmem = tmem_base + h * TN2;
-              const uint32_t a_off = h * (128 * TK2 * 2);  // second sub-tile: rows 128..255 of the K* boxes
-              const uint64_t a_hi = make_sdesc64(sa + a_off), a_lo = make_sdesc64(sa + TILE_BYTES2 + a_off);
-              const uint64_t b_hi = make_sdesc64(sa + 2 * TILE_BYTES2), b_lo = make_sdesc64(sa + 3 * TILE_BYTES2);
-#pragma unroll
-              for (int ks = 0; ks < TK2 / UK; ++ks) {
-                const uint64_t adv = (uint64_t)((ks * UK * 2) >> 4);
-                tc_mma_f16(d_tmem, a_hi + adv, b_hi + adv, IDESC, (kc | ks) ? 1u : 0u);
-                tc_mma_f16(d_tmem, a_hi + adv, b_lo + adv, IDESC, 1u);
-                tc_mma_f16(d_tmem, a_lo + adv, b_hi + adv, IDESC, 1u);
-              }
-            }
-            tc_commit(&empty[stage]);
-            if (++stage == STAGES2) {
-              stage = 0;
-              phase ^= 1u;
-            }
-          }
-          tc_commit(acc_full);
-          acc_phase ^= 1u;
-        }
-      }
-    }
-  } else {
-    const int quarter = warp & 3;
-    uint32_t acc_phase = 0;
-    for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
-      const int z = w & 1, wp = w >> 1;
-      const int m = wp / prm.n_pb, pb = wp - m * prm.n_pb;
-      const float* isc = prm.inv_scale + (int64_t)m * prm.l_rows;
-      const int j0 = z ? prm.j_split : 0, j1 = z ? prm.n_jt : prm.j_split;
-      double total0 = 0.0, total1 = 0.0;
-      for (int jt = j0; jt < j1; ++jt) {
-        mbar_wait(acc_full, acc_phase, abort_flag);
-        tc_fence_after();
-        float part0 = 0.f, part1 = 0.f;
-#pragma unroll 1
-        for (int c0 = 0; c0 < TN2; c0 += 32) {
-          uint32_t r0[32], r1[32];
-          const uint32_t t_addr = tmem_base + ((uint32_t)(quarter * 32) << 16) + c0;
-          tc_ld_32x32(t_addr, r0);
-          tc_ld_32x32(t_addr + TN2, r1);
-          tc_wait_ld();
-          const float* sc = isc + jt * TN2 + c0;
-#pragma unroll
-          for (int e = 0; e < 32; ++e) {
-            const float s = __ldg(sc + e);
-            const float t0 = __uint_as_float(r0[e]) * s, t1 = __uint_as_float(r1[e]) * s;
-            part0 = fmaf(t0, t0, part0);
-            part1 = fmaf(t1, t1, part1);
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(acc_empty);
-        total0 += (double)part0;
-        total1 += (double)part1;
-        acc_phase ^= 1u;
-      }
-      double* out = prm.vnorm + ((int64_t)z * prm.M + m) * prm.vn_ld + (int64_t)pb * TM2 + quarter * 32 + lane;
-      out[0] = total0;
-      out[128] = total1;
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
-}
-}  // namespace v2
-
-// ------------------------------------------------------------------------------------------------ the GEMM, version 3
-// Same tiles and pipeline as version 2; what changes is the work list and where K_* comes from.
+// ------------------------------------------------------------------------------------------------ the GEMM
+// The 256 candidates of a work item are two M = 128 sub-tiles that share every Linv tile, each with its own TMEM
+// accumulator (2 x 256 columns).  k is staged 32 elements at a time (64-byte rows, SWIZZLE_64B), so that three 64 KiB
+// stages fit.
 //   * A work item is (objective, 256 candidates, PAIR of Linv row blocks {q, n_jt - 1 - q}): every item costs the same
 //     n_jt + 1 k-blocks, so a static round-robin over the persistent CTAs has a tail of at most one item in
 //     M * n_pb * ceil(n_jt / 2) (6144 at the BASELINE shape, 41.5 rounds on 148 SMs).
 //   * Items are ordered (objective, candidate block, pair): the ceil(n_jt / 2) CTAs that hold the same candidate block
 //     start together at k = 0 and walk k at the same (MMA-bound) rate, so one of them pulls a K_* tile from DRAM and the
-//     others hit it in L2; version 2 ran 148 different candidate blocks at once and re-read every K_* tile from DRAM
-//     once per row block (22.6 GB per launch for 3.2 GB of operands).
-//   * Optional (DMO_GP_OVERLAP=1, off by default -- measured slower under the 1 kW power cap, see gp_predict_tensor): the
-//     kernel can be launched while the K_* producer (kstar_tensor_kernel, on the context's second stream) is still
-//     running; the TMA thread then waits for the producer's per-candidate-block completion counter before the first
-//     load of an item (ld.acquire.gpu + fence.proxy.async).
+//     others hit it in L2; inside an item the short row block goes first, so its K_* tiles are read again by the long one
+//     right away.
 namespace v3 {
-using v2::make_sdesc64;
-using v2::STAGE_BYTES2;
-using v2::STAGES2;
-using v2::TILE_BYTES2;
-using v2::TK2;
-using v2::TM2;
-using v2::TN2;
-using v2::GEMM_SMEM2;
+constexpr int BM = 256, BN = 256, BK = 32, STAGES = 3;  // candidates per item, Linv rows per row block, k per stage
+constexpr int TILE_BYTES = 256 * BK * 2;                // 16 KiB: 256 rows x 64 B
+constexpr int STAGE_BYTES = 4 * TILE_BYTES;             // K* hi/lo + Linv hi/lo
+constexpr size_t GEMM_SMEM = (size_t)STAGES * STAGE_BYTES + 1024 + 256;
+
+// K-major SWIZZLE_64B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor, mma_sm100_desc.hpp):
+//   [0,14) start address >> 4 | [16,30) leading byte offset >> 4 (unused for swizzled K-major: 1)
+//   [32,46) stride byte offset >> 4 (8 rows x 64 B = 512 B between 8-row groups) | [46,48) version = 1
+//   [61,64) layout type = 4 (SWIZZLE_64B)
+__device__ __forceinline__ uint64_t make_sdesc64(uint32_t smem_addr) {
+  return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | (1ull << 16) | ((uint64_t)(512 >> 4) << 32) | (1ull << 46) | (4ull << 61);
+}
 
 struct GemmParams3 {
   int M, n_pb, n_jt, n_q;
@@ -340,18 +156,7 @@ struct GemmParams3 {
   double* vnorm;  // [n_q][M][vn_ld]
   int64_t vn_ld;
   int* abort_flag;
-  const float* zf;        // [M][l_rows] whitened targets (nullptr: the mean is not taken from this contraction)
-  double* mnorm;          // [n_q][M][vn_ld] partial sums of D z
-  const unsigned* ready;  // [n_pb] completion counters of the K_* producer (nullptr: K_* is complete at launch)
-  unsigned ready_target;
-  int dbg;  // DMO_GP_DBG bits (diagnostics): 1 = no proxy fence, 2 = no nanosleep in the wait loop
 };
-
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
 
 __global__ void __launch_bounds__(NTHREADS, 1)
     gp_var_tc3_kernel(const __grid_constant__ CUtensorMap map_kh, const __grid_constant__ CUtensorMap map_kl,
@@ -359,17 +164,17 @@ __global__ void __launch_bounds__(NTHREADS, 1)
                       const GemmParams3 prm) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* tiles = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  uint64_t* bars = (uint64_t*)(tiles + (size_t)STAGES2 * STAGE_BYTES2);
+  uint64_t* bars = (uint64_t*)(tiles + (size_t)STAGES * STAGE_BYTES);
   uint64_t* full = bars;
-  uint64_t* empty = bars + STAGES2;
-  uint64_t* acc_full = bars + 2 * STAGES2;
-  uint64_t* acc_empty = bars + 2 * STAGES2 + 1;
-  uint32_t* tmem_slot = (uint32_t*)(bars + 2 * STAGES2 + 2);
+  uint64_t* empty = bars + STAGES;
+  uint64_t* acc_full = bars + 2 * STAGES;
+  uint64_t* acc_empty = bars + 2 * STAGES + 1;
+  uint32_t* tmem_slot = (uint32_t*)(bars + 2 * STAGES + 2);
   volatile int* abort_flag = prm.abort_flag;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < STAGES2; ++s) {
+    for (int s = 0; s < STAGES; ++s) {
       mbar_init(&full[s], 1);
       mbar_init(&empty[s], 1);
     }
@@ -395,36 +200,22 @@ __global__ void __launch_bounds__(NTHREADS, 1)
       for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
         const int m = w / per_m, r = w - m * per_m;
         const int pb = r / prm.n_q, q = r - pb * prm.n_q;
-        if (prm.ready) {  // the K_* rows of this candidate block must have been written (by another kernel, generic proxy)
-          uint32_t spins = 0;
-          while (ld_acquire_u32(prm.ready + pb) < prm.ready_target) {
-            if (!(prm.dbg & 2)) __nanosleep(256);
-            if ((++spins & 0xFFu) == 0u) {
-              if (*abort_flag) break;
-              if (spins > (1u << 23)) {  // ~2 s: the producer is not running
-                *abort_flag = 2;
-                break;
-              }
-            }
-          }
-          if (!(prm.dbg & 1)) asm volatile("fence.proxy.async;" ::: "memory");  // order the TMA (async proxy) reads after the acquire
-        }
-        const int a_row = (int)(m * prm.k_rows + (int64_t)pb * TM2);
+        const int a_row = (int)(m * prm.k_rows + (int64_t)pb * BM);
         const int jhi = prm.n_jt - 1 - q;
         for (int s = 0; s < 2; ++s) {  // short row block first: its K_* tiles are read again right away by the long one
           const int jt = s ? jhi : q;
           if (s && q == jhi) break;
-          const int b_row = (int)(m * prm.l_rows + (int64_t)jt * TN2);
-          const int nkc = (jt + 1) * (TN2 / TK2);
+          const int b_row = (int)(m * prm.l_rows + (int64_t)jt * BN);
+          const int nkc = (jt + 1) * (BN / BK);
           for (int kc = 0; kc < nkc; ++kc) {
             mbar_wait(&empty[stage], phase ^ 1u, abort_flag);
-            uint8_t* st = tiles + (size_t)stage * STAGE_BYTES2;
-            mbar_expect_tx(&full[stage], STAGE_BYTES2);
-            tma_load_2d(&map_kh, &full[stage], st, kc * TK2, a_row);
-            tma_load_2d(&map_kl, &full[stage], st + TILE_BYTES2, kc * TK2, a_row);
-            tma_load_2d(&map_lh, &full[stage], st + 2 * TILE_BYTES2, kc * TK2, b_row);
-            tma_load_2d(&map_ll, &full[stage], st + 3 * TILE_BYTES2, kc * TK2, b_row);
-            if (++stage == STAGES2) {
+            uint8_t* st = tiles + (size_t)stage * STAGE_BYTES;
+            mbar_expect_tx(&full[stage], STAGE_BYTES);
+            tma_load_2d(&map_kh, &full[stage], st, kc * BK, a_row);
+            tma_load_2d(&map_kl, &full[stage], st + TILE_BYTES, kc * BK, a_row);
+            tma_load_2d(&map_lh, &full[stage], st + 2 * TILE_BYTES, kc * BK, b_row);
+            tma_load_2d(&map_ll, &full[stage], st + 3 * TILE_BYTES, kc * BK, b_row);
+            if (++stage == STAGES) {
               stage = 0;
               phase ^= 1u;
             }
@@ -444,19 +235,19 @@ __global__ void __launch_bounds__(NTHREADS, 1)
           if (s && q == jhi) break;
           mbar_wait(acc_empty, acc_phase ^ 1u, abort_flag);
           tc_fence_after();
-          const int nkc = (jt + 1) * (TN2 / TK2);
+          const int nkc = (jt + 1) * (BN / BK);
           for (int kc = 0; kc < nkc; ++kc) {
             mbar_wait(&full[stage], phase, abort_flag);
             tc_fence_after();
-            const uint32_t sa = smem_u32(tiles + (size_t)stage * STAGE_BYTES2);
+            const uint32_t sa = smem_u32(tiles + (size_t)stage * STAGE_BYTES);
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
-              const uint32_t d_tmem = tmem_base + h * TN2;
-              const uint32_t a_off = h * (128 * TK2 * 2);
-              const uint64_t a_hi = make_sdesc64(sa + a_off), a_lo = make_sdesc64(sa + TILE_BYTES2 + a_off);
-              const uint64_t b_hi = make_sdesc64(sa + 2 * TILE_BYTES2), b_lo = make_sdesc64(sa + 3 * TILE_BYTES2);
+              const uint32_t d_tmem = tmem_base + h * BN;
+              const uint32_t a_off = h * (128 * BK * 2);  // second sub-tile: rows 128..255 of the K* boxes
+              const uint64_t a_hi = make_sdesc64(sa + a_off), a_lo = make_sdesc64(sa + TILE_BYTES + a_off);
+              const uint64_t b_hi = make_sdesc64(sa + 2 * TILE_BYTES), b_lo = make_sdesc64(sa + 3 * TILE_BYTES);
 #pragma unroll
-              for (int ks = 0; ks < TK2 / UK; ++ks) {
+              for (int ks = 0; ks < BK / UK; ++ks) {
                 const uint64_t adv = (uint64_t)((ks * UK * 2) >> 4);
                 tc_mma_f16(d_tmem, a_hi + adv, b_hi + adv, IDESC, (kc | ks) ? 1u : 0u);
                 tc_mma_f16(d_tmem, a_hi + adv, b_lo + adv, IDESC, 1u);
@@ -464,7 +255,7 @@ __global__ void __launch_bounds__(NTHREADS, 1)
               }
             }
             tc_commit(&empty[stage]);
-            if (++stage == STAGES2) {
+            if (++stage == STAGES) {
               stage = 0;
               phase ^= 1u;
             }
@@ -481,47 +272,30 @@ __global__ void __launch_bounds__(NTHREADS, 1)
       const int m = w / per_m, r = w - m * per_m;
       const int pb = r / prm.n_q, q = r - pb * prm.n_q;
       const float* isc = prm.inv_scale + (int64_t)m * prm.l_rows;
-      const float* zf = prm.zf ? prm.zf + (int64_t)m * prm.l_rows : nullptr;
       const int jhi = prm.n_jt - 1 - q;
-      double total0 = 0.0, total1 = 0.0, mtot0 = 0.0, mtot1 = 0.0;
+      double total0 = 0.0, total1 = 0.0;
       for (int s = 0; s < 2; ++s) {
         const int jt = s ? jhi : q;
         if (s && q == jhi) break;
         mbar_wait(acc_full, acc_phase, abort_flag);
         tc_fence_after();
 #pragma unroll 1
-        for (int c0 = 0; c0 < TN2; c0 += 32) {
+        for (int c0 = 0; c0 < BN; c0 += 32) {
           uint32_t r0[32], r1[32];
           const uint32_t t_addr = tmem_base + ((uint32_t)(quarter * 32) << 16) + c0;
           tc_ld_32x32(t_addr, r0);
-          tc_ld_32x32(t_addr + TN2, r1);
+          tc_ld_32x32(t_addr + BN, r1);
           tc_wait_ld();
-          const float* sc = isc + jt * TN2 + c0;
+          const float* sc = isc + jt * BN + c0;
           // four independent fp32 partial sums per sub-tile over 8 squares each, folded into float64 every 32 columns:
           // the rounding of the sum of squares stays at the 2^-24 * sqrt(8) level instead of growing with N
           float p0[4] = {0.f, 0.f, 0.f, 0.f}, p1[4] = {0.f, 0.f, 0.f, 0.f};
-          if (zf) {  // posterior mean = D z out of the same accumulator (z = L^-1 y_n): one more FMA per element
-            const float* zc = zf + jt * TN2 + c0;
-            float q0[4] = {0.f, 0.f, 0.f, 0.f}, q1[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
-            for (int e = 0; e < 32; ++e) {
-              const float sv = __ldg(sc + e), zv = __ldg(zc + e);
-              const float t0 = __uint_as_float(r0[e]) * sv, t1 = __uint_as_float(r1[e]) * sv;
-              p0[e & 3] = fmaf(t0, t0, p0[e & 3]);
-              p1[e & 3] = fmaf(t1, t1, p1[e & 3]);
-              q0[e & 3] = fmaf(t0, zv, q0[e & 3]);
-              q1[e & 3] = fmaf(t1, zv, q1[e & 3]);
-            }
-            mtot0 += ((double)q0[0] + (double)q0[1]) + ((double)q0[2] + (double)q0[3]);
-            mtot1 += ((double)q1[0] + (double)q1[1]) + ((double)q1[2] + (double)q1[3]);
-          } else {
-#pragma unroll
-            for (int e = 0; e < 32; ++e) {
-              const float sv = __ldg(sc + e);
-              const float t0 = __uint_as_float(r0[e]) * sv, t1 = __uint_as_float(r1[e]) * sv;
-              p0[e & 3] = fmaf(t0, t0, p0[e & 3]);
-              p1[e & 3] = fmaf(t1, t1, p1[e & 3]);
-            }
+          for (int e = 0; e < 32; ++e) {
+            const float sv = __ldg(sc + e);
+            const float t0 = __uint_as_float(r0[e]) * sv, t1 = __uint_as_float(r1[e]) * sv;
+            p0[e & 3] = fmaf(t0, t0, p0[e & 3]);
+            p1[e & 3] = fmaf(t1, t1, p1[e & 3]);
           }
           total0 += ((double)p0[0] + (double)p0[1]) + ((double)p0[2] + (double)p0[3]);
           total1 += ((double)p1[0] + (double)p1[1]) + ((double)p1[2] + (double)p1[3]);
@@ -531,12 +305,7 @@ __global__ void __launch_bounds__(NTHREADS, 1)
         if (lane == 0) mbar_arrive(acc_empty);
         acc_phase ^= 1u;
       }
-      if (zf) {
-        double* mo = prm.mnorm + ((int64_t)q * prm.M + m) * prm.vn_ld + (int64_t)pb * TM2 + quarter * 32 + lane;
-        mo[0] = mtot0;
-        mo[128] = mtot1;
-      }
-      double* out = prm.vnorm + ((int64_t)q * prm.M + m) * prm.vn_ld + (int64_t)pb * TM2 + quarter * 32 + lane;
+      double* out = prm.vnorm + ((int64_t)q * prm.M + m) * prm.vn_ld + (int64_t)pb * BM + quarter * 32 + lane;
       out[0] = total0;
       out[128] = total1;
     }
@@ -624,7 +393,7 @@ __global__ void __launch_bounds__(KT_TN)
                         const double* __restrict__ Xt, int64_t N, int d, int M, int kind,
                         const double* __restrict__ inv_ls, const double* __restrict__ constant,
                         const int* __restrict__ k_exp, int64_t ldk, int64_t plane, uint16_t* __restrict__ Kh,
-                        uint16_t* __restrict__ Kl, unsigned* __restrict__ ready) {
+                        uint16_t* __restrict__ Kl) {
   extern __shared__ __align__(16) float sxf[];  // [KT_TP][DMAX] candidate tile, then [M][DMAX] 1/l, [M] c * 2^kexp
   float* s_il = sxf + KT_TP * DMAX;
   float* s_c = s_il + M * DMAX;
@@ -712,15 +481,6 @@ __global__ void __launch_bounds__(KT_TN)
       const int64_t o = (m * plane + pl * ldk + n0) >> 1;
       Kh32[o] = *reinterpret_cast<const uint32_t*>(&h);
       Kl32[o] = *reinterpret_cast<const uint32_t*>(&l);
-    }
-  }
-  if (ready) {
-    // publish this block's rows to the variance kernel that is already running (v3::gp_var_tc3_kernel): every thread's
-    // stores happen-before the barrier, the fence makes them visible at GPU scope before the counter moves
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      __threadfence();
-      atomicAdd(ready + pt0 / 256, 1u);
     }
   }
 }
@@ -1079,8 +839,8 @@ __global__ void mean_split_kernel(const uint16_t* __restrict__ Kh, const uint16_
   if (lane == 0) mean[(p_base + pl) * M + m] = ystd[m] * scalbn(s, -k_exp[m]) + ymean[m];
 }
 
-// mean[p][m] = y_std * sum over the work items' partial sums of D z + y_mean (fixed order)
-__global__ void mean_finish_tc_kernel(const double* __restrict__ mnorm, int nplanes, int64_t Pc, int64_t ld, int M,
+// mean[p][m] = y_std * sum over the training-set slices' partial sums of K_* alpha + y_mean (fixed order)
+__global__ void mean_finish_tc_kernel(const double* __restrict__ mpart, int nplanes, int64_t Pc, int64_t ld, int M,
                                       const double* __restrict__ ymean, const double* __restrict__ ystd, int64_t p_base,
                                       double* __restrict__ mean) {
   int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1088,7 +848,7 @@ __global__ void mean_finish_tc_kernel(const double* __restrict__ mnorm, int npla
   int64_t pl = t / M;
   int m = (int)(t - pl * M);
   double s = 0.0;
-  for (int q = 0; q < nplanes; ++q) s += mnorm[((int64_t)q * M + m) * ld + pl];
+  for (int q = 0; q < nplanes; ++q) s += mpart[((int64_t)q * M + m) * ld + pl];
   mean[(p_base + pl) * M + m] = ystd[m] * s + ymean[m];
 }
 
@@ -1240,82 +1000,46 @@ int gp_mean_direct(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, doubl
 
 }  // namespace
 
-int gp_predict_tensor(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, double* d_mean, double* d_var, bool mean_from_d) {
+int gp_predict_tensor(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, double* d_mean, double* d_var) {
   const int64_t N = gp->N, Npad = gp->Npad;
   const int M = gp->M, d = gp->d;
   DMO_REQUIRE(M <= 16, "gp_predict(tensor): at most 16 objectives per model (got %d)", M);
   DMO_REQUIRE(d <= 64, "gp_predict(tensor): at most 64 input dimensions (got %d); use DMO_GP_FP64", d);
   DMO_REQUIRE(Npad % TN == 0, "gp_predict(tensor): internal padding error");
-  if (!d_var && d <= KM_D && M <= 6 && !(getenv("DMO_GP_MEAN_DIRECT") && atoi(getenv("DMO_GP_MEAN_DIRECT")) == 0))
+  if (!d_var && d <= KM_D && M <= 6)
     return gp_mean_direct(ctx, gp, dXn, P, d_mean);  // nothing but the mean is wanted: K_* stays in registers
   DMO_TRY(prepare_tensor_state(ctx, gp));
-  // kernel version: 3 (default) = equal-cost paired row blocks in L2-friendly order, overlapped with the K_* producer;
-  // 2 = previous schedule, K_* / mean / variance back to back on one stream (DMO_GP_TC=2, kept for comparison)
-  int version = 3;
-  if (const char* e = getenv("DMO_GP_TC")) version = atoi(e) == 2 ? 2 : 3;
-  // DMO_GP_OVERLAP=1 (experimental, off by default): launch the contraction while the K_* producer is still running on
-  // the context's second stream and let its TMA thread wait on per-candidate-block completion counters.  Measured on
-  // B200 (profiles/README.md, round 2): no gain -- the contraction is power-capped, co-running FP32 work lowers its clock
-  // by what the overlap hides (10.35 ms vs 9.98 ms per predict at P = 65 536) -- and the co-residency of the two kernels
-  // is not guaranteed by the hardware scheduler (a launch at P = 4608 failed), so the in-line order is the product path.
-  const bool overlap = version == 3 && getenv("DMO_GP_OVERLAP") && atoi(getenv("DMO_GP_OVERLAP"));
-  const int dbg = getenv("DMO_GP_DBG") ? atoi(getenv("DMO_GP_DBG")) : 0;  // 4: event instead of flags, 8: mean after var
-  const bool use_flags = overlap && !(dbg & 4);
-  // mean from the contraction (D z) instead of the K_* alpha pass: only with the variance, version 3 and a model created from L
-  mean_from_d = mean_from_d && d_var != nullptr && version == 3 && gp->z_ready;
-  constexpr int64_t TMv = v2::TM2;
+  constexpr int64_t BM = v3::BM;
   // candidate chunk: K_* hi/lo (2 x M x Pc x Npad fp16) within ~6 GiB
   int64_t Pc_max = ((int64_t)6 << 30) / ((int64_t)M * Npad * 4);
-  Pc_max = (Pc_max / TMv) * TMv;
-  if (Pc_max < TMv) Pc_max = TMv;
-  const int64_t Pc_alloc = P < Pc_max ? ceil_div(P, TMv) * TMv : Pc_max;
-  const int n_jt = (int)(Npad / v2::TN2);
-  const int n_q = version == 3 ? (n_jt + 1) / 2 : 2;
-  const int64_t n_chunks = ceil_div(P, Pc_alloc);
-  const int n_pb_alloc = (int)(Pc_alloc / TMv);
+  Pc_max = (Pc_max / BM) * BM;
+  if (Pc_max < BM) Pc_max = BM;
+  const int64_t Pc_alloc = P < Pc_max ? ceil_div(P, BM) * BM : Pc_max;
+  const int n_jt = (int)(Npad / v3::BN);
+  const int n_q = (n_jt + 1) / 2;
   DevBuf<uint16_t> Kh, Kl;
   DevBuf<double> vnorm;
   DevBuf<int> abort_flag;
-  DevBuf<unsigned> ready;
   DMO_TRY(Kh.alloc(ctx, (size_t)M * Pc_alloc * Npad));
   DMO_TRY(Kl.alloc(ctx, (size_t)M * Pc_alloc * Npad));
   DMO_TRY(vnorm.alloc(ctx, (size_t)n_q * M * Pc_alloc));
-  DevBuf<double> mnorm;
-  if (mean_from_d) DMO_TRY(mnorm.alloc(ctx, (size_t)n_q * M * Pc_alloc));
   DMO_TRY(abort_flag.alloc(ctx, 1));
-  DMO_TRY(ready.alloc(ctx, (size_t)n_chunks * n_pb_alloc));
   DMO_CUDA(cudaMemsetAsync(abort_flag.p, 0, sizeof(int), ctx->stream));
-  DMO_CUDA(cudaMemsetAsync(ready.p, 0, (size_t)n_chunks * n_pb_alloc * sizeof(unsigned), ctx->stream));
   CUtensorMap map_kh, map_kl, map_lh, map_ll;
-  DMO_TRY(make_map(ctx, &map_kh, Kh.p, (uint64_t)M * Pc_alloc, (uint64_t)Npad, 256, v2::TK2, CU_TENSOR_MAP_SWIZZLE_64B));
-  DMO_TRY(make_map(ctx, &map_kl, Kl.p, (uint64_t)M * Pc_alloc, (uint64_t)Npad, 256, v2::TK2, CU_TENSOR_MAP_SWIZZLE_64B));
-  DMO_TRY(make_map(ctx, &map_lh, gp->Lhi.p, (uint64_t)M * Npad, (uint64_t)Npad, 256, v2::TK2, CU_TENSOR_MAP_SWIZZLE_64B));
-  DMO_TRY(make_map(ctx, &map_ll, gp->Llo.p, (uint64_t)M * Npad, (uint64_t)Npad, 256, v2::TK2, CU_TENSOR_MAP_SWIZZLE_64B));
-  DMO_CUDA(cudaFuncSetAttribute(v2::gp_var_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)v2::GEMM_SMEM2));
-  DMO_CUDA(cudaFuncSetAttribute(v3::gp_var_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)v2::GEMM_SMEM2));
+  DMO_TRY(make_map(ctx, &map_kh, Kh.p, (uint64_t)M * Pc_alloc, (uint64_t)Npad, 256, v3::BK, CU_TENSOR_MAP_SWIZZLE_64B));
+  DMO_TRY(make_map(ctx, &map_kl, Kl.p, (uint64_t)M * Pc_alloc, (uint64_t)Npad, 256, v3::BK, CU_TENSOR_MAP_SWIZZLE_64B));
+  DMO_TRY(make_map(ctx, &map_lh, gp->Lhi.p, (uint64_t)M * Npad, (uint64_t)Npad, 256, v3::BK, CU_TENSOR_MAP_SWIZZLE_64B));
+  DMO_TRY(make_map(ctx, &map_ll, gp->Llo.p, (uint64_t)M * Npad, (uint64_t)Npad, 256, v3::BK, CU_TENSOR_MAP_SWIZZLE_64B));
+  DMO_CUDA(cudaFuncSetAttribute(v3::gp_var_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)v3::GEMM_SMEM));
   const int64_t kplane = Pc_alloc * Npad;
-  // K_* producer fused with the mean (d <= 32, M <= 6; DMO_GP_FUSED=0 keeps kstar_tensor_kernel + mean_split_kernel)
-  // (per-dimension length scales with more than two objectives spill in the fused kernel: they keep the two-kernel route)
-  const bool fused = !overlap && !mean_from_d && !(dbg & 8) && d <= KM_D && M <= 6 && (gp->isotropic || M <= 2) &&
-                     !(getenv("DMO_GP_FUSED") && atoi(getenv("DMO_GP_FUSED")) == 0);
+  // K_* producer fused with the mean (d <= 32, M <= 6); per-dimension length scales with more than two objectives spill
+  // in the fused kernel, so they take kstar_tensor_kernel + mean_split_kernel like the shapes it does not take at all
+  const bool fused = d <= KM_D && M <= 6 && (gp->isotropic || M <= 2);
   DevBuf<double> mpart;
   if (fused) DMO_TRY(prepare_direct_state(ctx, gp));
-  // producer side (K_* and the mean) on the second stream when overlapping, else in line
-  cudaStream_t ps = overlap ? ctx->aux : ctx->stream;
-  if (overlap) {
-    DMO_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));  // allocations, memsets and Xn are ready
-    DMO_CUDA(cudaStreamWaitEvent(ctx->aux, ctx->ev_fork, 0));
-  }
-  int64_t chunk = 0;
-  for (int64_t p_base = 0; p_base < P; p_base += Pc_alloc, ++chunk) {
+  for (int64_t p_base = 0; p_base < P; p_base += Pc_alloc) {
     const int64_t Pc = (P - p_base) < Pc_alloc ? (P - p_base) : Pc_alloc;
-    const int64_t Pcpad = ceil_div(Pc, TMv) * TMv;
-    unsigned* rdy = ready.p + chunk * n_pb_alloc;
-    dim3 gk((unsigned)(Npad / (2 * KT_TN)), (unsigned)ceil_div(Pcpad, KT_TP));
-    if (overlap && chunk > 0) {  // the K_* buffers are reused: the previous chunk's contraction must have drained them
-      DMO_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
-      DMO_CUDA(cudaStreamWaitEvent(ctx->aux, ctx->ev_fork, 0));
-    }
+    const int64_t Pcpad = ceil_div(Pc, BM) * BM;
     if (fused) {
       // K_* and the mean from one kernel (kstar_mean_kernel): K_* is written once and never read back for the mean
       int64_t n_per_block = Npad;
@@ -1352,14 +1076,14 @@ int gp_predict_tensor(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, do
       DMO_LAUNCH(mean_finish_tc_kernel, (unsigned)ceil_div(Pc * M, 256), 256, 0, mpart.p, (int)nsplit, Pc, Pcpad, M, gp->ymean.p,
                  gp->ystd.p, p_base, d_mean);
     } else {
-    {
-        ProfileScope ps_(ctx, "gp_kstar", ps);
+      {
+        ProfileScope ps_(ctx, "gp_kstar");
+        dim3 gk((unsigned)(Npad / (2 * KT_TN)), (unsigned)ceil_div(Pcpad, KT_TP));
         const int dmax = d <= 32 ? 32 : 64;
         size_t smem = (size_t)(KT_TP * dmax + M * dmax + M) * sizeof(float);
-  #define KSTAR_LAUNCH(ISO_, DM_)                                                                                   \
-    DMO_LAUNCH_ON(ps, (kstar_tensor_kernel<ISO_, DM_>), gk, KT_TN, smem, dXn, P, p_base, Pcpad, gp->Xt.p, N, d, M,    \
-                  gp->kernel, gp->inv_ls.p, gp->constant.p, gp->Kexp.p, Npad, kplane, Kh.p, Kl.p,                    \
-                  (use_flags && d_var) ? rdy : nullptr)
+#define KSTAR_LAUNCH(ISO_, DM_)                                                                                 \
+  DMO_LAUNCH((kstar_tensor_kernel<ISO_, DM_>), gk, KT_TN, smem, dXn, P, p_base, Pcpad, gp->Xt.p, N, d, M, gp->kernel, \
+             gp->inv_ls.p, gp->constant.p, gp->Kexp.p, Npad, kplane, Kh.p, Kl.p)
         if (gp->isotropic) {
           if (d <= 32)
             KSTAR_LAUNCH(true, 32);
@@ -1371,23 +1095,18 @@ int gp_predict_tensor(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, do
           else
             KSTAR_LAUNCH(false, 64);
         }
-  #undef KSTAR_LAUNCH
+#undef KSTAR_LAUNCH
       }
-      if (overlap && (dbg & 4)) {  // diagnostics: the contraction waits for the whole K_* kernel by event, the mean still overlaps
-        DMO_CUDA(cudaEventRecord(ctx->ev_fork, ctx->aux));
-        DMO_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_fork, 0));
+      {
+        ProfileScope ps_(ctx, "gp_mean");
+        DMO_LAUNCH(mean_split_kernel, (unsigned)ceil_div(Pc * M * 32, 256), 256, 0, Kh.p, Kl.p, Pc, N, Npad, kplane, M,
+                   gp->Kexp.p, gp->alpha.p, gp->ymean.p, gp->ystd.p, p_base, d_mean);
       }
-      if (!(dbg & 8) && !mean_from_d) {
-        ProfileScope ps_(ctx, "gp_mean", ps);
-        DMO_LAUNCH_ON(ps, mean_split_kernel, (unsigned)ceil_div(Pc * M * 32, 256), 256, 0, Kh.p, Kl.p, Pc, N, Npad, kplane,
-                      M, gp->Kexp.p, gp->alpha.p, gp->ymean.p, gp->ystd.p, p_base, d_mean);
-      }
-}
-    if (overlap) DMO_CUDA(cudaEventRecord(ctx->ev_join, ctx->aux));
-    if (d_var && version == 3) {
+    }
+    if (d_var) {
       v3::GemmParams3 prm;
       prm.M = M;
-      prm.n_pb = (int)(Pcpad / TMv);
+      prm.n_pb = (int)(Pcpad / BM);
       prm.n_jt = n_jt;
       prm.n_q = n_q;
       prm.k_rows = Pc_alloc;
@@ -1396,69 +1115,20 @@ int gp_predict_tensor(dmo_ctx* ctx, dmo_gp* gp, const double* dXn, int64_t P, do
       prm.vnorm = vnorm.p;
       prm.vn_ld = Pc_alloc;
       prm.abort_flag = abort_flag.p;
-      prm.zf = mean_from_d ? gp->Zf.p : nullptr;
-      prm.mnorm = mean_from_d ? mnorm.p : nullptr;
-      prm.ready = use_flags ? rdy : nullptr;
-      prm.dbg = dbg;
-      prm.ready_target = 8u * gk.x;  // KT_TP = 32 candidates per producer block: 8 tile rows x gk.x column blocks per 256
       const int n_work = prm.M * prm.n_pb * prm.n_q;
       const int grid = n_work < ctx->sm_count ? n_work : ctx->sm_count;
       {
         ProfileScope ps_(ctx, "gp_var");
-        DMO_LAUNCH(v3::gp_var_tc3_kernel, grid, NTHREADS, v2::GEMM_SMEM2, map_kh, map_kl, map_lh, map_ll, prm);
+        DMO_LAUNCH(v3::gp_var_tc3_kernel, grid, NTHREADS, v3::GEMM_SMEM, map_kh, map_kl, map_lh, map_ll, prm);
       }
       DMO_LAUNCH(var_finish_tc_kernel, (unsigned)ceil_div(Pc * M, 256), 256, 0, vnorm.p, n_q, Pc, Pc_alloc, M,
                  gp->constant.p, gp->noise.p, gp->ystd.p, p_base, d_var);
-      if (mean_from_d)
-        DMO_LAUNCH(mean_finish_tc_kernel, (unsigned)ceil_div(Pc * M, 256), 256, 0, mnorm.p, n_q, Pc, Pc_alloc, M, gp->ymean.p,
-                   gp->ystd.p, p_base, d_mean);
-    } else if (d_var) {
-      v2::GemmParams2 prm;
-      prm.M = M;
-      prm.n_pb = (int)(Pcpad / v2::TM2);
-      prm.n_jt = n_jt;
-      // split the row blocks where the cumulative MMA count sum_{j < J} (j + 1) is closest to half of the total
-      {
-        const int64_t tot = (int64_t)prm.n_jt * (prm.n_jt + 1) / 2;
-        int best_j = prm.n_jt;
-        int64_t best_d = tot;
-        for (int J = 0; J <= prm.n_jt; ++J) {
-          const int64_t dlt = llabs(2 * ((int64_t)J * (J + 1) / 2) - tot);
-          if (dlt < best_d) {
-            best_d = dlt;
-            best_j = J;
-          }
-        }
-        prm.j_split = best_j;
-      }
-      prm.k_rows = Pc_alloc;
-      prm.l_rows = Npad;
-      prm.inv_scale = gp->Lscale.p;
-      prm.vnorm = vnorm.p;
-      prm.vn_ld = Pc_alloc;
-      prm.abort_flag = abort_flag.p;
-      const int n_work = prm.M * prm.n_pb * 2;
-      const int grid = n_work < ctx->sm_count ? n_work : ctx->sm_count;
-      {
-        ProfileScope ps_(ctx, "gp_var");
-        DMO_LAUNCH(v2::gp_var_tc2_kernel, grid, NTHREADS, v2::GEMM_SMEM2, map_kh, map_kl, map_lh, map_ll, prm);
-      }
-      DMO_LAUNCH(var_finish_tc_kernel, (unsigned)ceil_div(Pc * M, 256), 256, 0, vnorm.p, 2, Pc, Pc_alloc, M,
-                 gp->constant.p, gp->noise.p, gp->ystd.p, p_base, d_var);
-    }
-    if (overlap) DMO_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));  // mean (and K_*) of this chunk done
-    if ((dbg & 8) && !mean_from_d) {
-      ProfileScope ps_(ctx, "gp_mean");
-      DMO_LAUNCH(mean_split_kernel, (unsigned)ceil_div(Pc * M * 32, 256), 256, 0, Kh.p, Kl.p, Pc, N, Npad, kplane, M,
-                 gp->Kexp.p, gp->alpha.p, gp->ymean.p, gp->ystd.p, p_base, d_mean);
     }
   }
   DMO_CHECK_LAUNCH();
   int h_abort = 0;
   DMO_CUDA(cudaMemcpyAsync(&h_abort, abort_flag.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   DMO_CUDA(cudaStreamSynchronize(ctx->stream));
-  if (h_abort)
-    return dmo_fail(ctx, DMO_ERR_INTERNAL, "gp_predict(tensor): pipeline watchdog tripped (%s)",
-                    h_abort == 2 ? "K_* producer did not deliver" : "mbarrier wait timed out");
+  if (h_abort) return dmo_fail(ctx, DMO_ERR_INTERNAL, "gp_predict(tensor): pipeline watchdog tripped (mbarrier wait timed out)");
   return DMO_OK;
 }

@@ -216,9 +216,9 @@ int dmo_gp_predict(dmo_ctx* ctx, dmo_gp* gp, const double* X, int64_t P, double*
                    double* var, int precision);
 /* What DMO_GP_AUTO decided for this model (runs the one-off calibration if it has not run yet):
  * both arithmetic paths predict 512 probe candidates; mean_tensor bit 0 = the fp32-K_* alpha pass is
- * admitted (predicts with variance), bit 1 = the mean is taken from the variance contraction (D z, predicts with
- * variance), bit 2 = the mean-only kernel (K_* never written, fp32 kernel values, float64 partial sums) is admitted
- * for predicts without variance; var_tensor = 1 when the tcgen05 variance is admitted; errors relative to max(|mean|, y_std) and to
+ * admitted (predicts with variance), bit 1 is reserved (always 0), bit 2 = the mean-only kernel (K_* never
+ * written, fp32 kernel values, float64 partial sums) is admitted for predicts without variance;
+ * var_tensor = 1 when the tcgen05 variance is admitted; errors relative to max(|mean|, y_std) and to
  * the prior variance, margins documented in csrc/gp.cu; theta: rows whose tensor variance is
  * below theta * prior are recomputed in float64; last_refined: rows the last AUTO predict recomputed
  * (= P when the whole call ran in float64).  Any output pointer may be NULL. */

@@ -41,7 +41,7 @@ def main():
 
 
 def gp_sweep():
-    """GP posterior at the BASELINE shape: fp64 vs tensor path versions (DMO_GP_TC=1|2), accuracy and time."""
+    """GP posterior at the BASELINE shape: fp64 vs tensor path, accuracy and time."""
     L.context()
     rng = np.random.default_rng(1)
     N, d, M, P = 4096, 30, 3, 65536
@@ -71,7 +71,7 @@ def gp_sweep():
         else:
             err = f" | vs fp64: var err/prior {np.max(np.abs(var - ref[1]) / prior):.2e}, mean err {np.max(np.abs(mean - ref[0])):.2e}"
         parts = ", ".join(f"{k} {v[0] / v[1]:.3f}" for k, v in rep.items())
-        print(f"gp {name} (DMO_GP_TC={os.environ.get('DMO_GP_TC', 'default')}): total {ms:.3f} ms [{parts}]{err}", flush=True)
+        print(f"gp {name}: total {ms:.3f} ms [{parts}]{err}", flush=True)
 
 
 def stream_sweep():

@@ -307,25 +307,31 @@ def test_gp_predict_baseline_shape_vs_oracle(L):
     h.close()
 
 
-def _baseline_gp(N, d, M, seed):
+def _baseline_gp(N, d, M, seed, ard=False):
     rng = np.random.default_rng(seed)
     xlb, xub = np.zeros(d), np.ones(d)
     Xtr = rng.random((N, d))
     Ytr = np.column_stack([np.sin(3 * Xtr[:, :4].sum(axis=1) + k) + Xtr[:, 4 + k] ** 2 for k in range(M)])
-    st = gp.fit_fixed(Xtr, Ytr, xlb, xub, 1.0, 0.5, 1e-6)
+    ls = [0.3 + 0.5 * rng.random(d) for _ in range(M)] if ard else 0.5  # per-dimension length scales per objective
+    st = gp.fit_fixed(Xtr, Ytr, xlb, xub, 1.0, ls, 1e-6)
     return rng, xlb, xub, Xtr, st
 
 
 def _handle_from_state(L, st, d):
     return L.GPHandle(st.X_train, np.stack([o.alpha for o in st.objectives]), np.stack([o.L for o in st.objectives]), [o.constant for o in st.objectives],
-                      [np.full(d, float(o.length_scale)) for o in st.objectives], [o.noise for o in st.objectives], [o.y_mean for o in st.objectives],
-                      [o.y_std for o in st.objectives], st.xlb, st.xub)
+                      [np.broadcast_to(np.asarray(o.length_scale, dtype=np.float64), (d,)) for o in st.objectives], [o.noise for o in st.objectives],
+                      [o.y_mean for o in st.objectives], [o.y_std for o in st.objectives], st.xlb, st.xub)
 
 
-@pytest.mark.parametrize("N,d,M,P", [(300, 30, 3, 200), (1000, 12, 2, 517), (2048, 30, 3, 1500), (600, 22, 5, 700)])
-def test_gp_predict_tensor_path(L, N, d, M, P):
+# The last three shapes take kstar_tensor_kernel + mean_split_kernel instead of the fused K_* + mean kernel: per-dimension
+# length scales with three objectives, d > 32 (the DMAX = 64 instantiation) and M > 6.
+@pytest.mark.parametrize("N,d,M,P,ard", [
+    pytest.param(*c, id="-".join(map(str, c[:4])) + ("-ard" if c[4] else ""))
+    for c in [(300, 30, 3, 200, False), (1000, 12, 2, 517, False), (2048, 30, 3, 1500, False), (600, 22, 5, 700, False),
+              (1000, 30, 3, 900, True), (1100, 48, 2, 700, False), (700, 16, 7, 600, False)]])
+def test_gp_predict_tensor_path(L, N, d, M, P, ard):
     """tcgen05 split-fp16 path: |var - var_ref| <= 1e-5 * prior variance, |mean - mean_ref| <= 1e-5 * max(|mean|, y_std)."""
-    rng, xlb, xub, Xtr, st = _baseline_gp(N, d, M, 100 + N)
+    rng, xlb, xub, Xtr, st = _baseline_gp(N, d, M, 100 + N, ard)
     X = rng.random((P, d))
     X[:6] = np.clip(Xtr[:6] + 2e-3 * rng.standard_normal((6, d)), 0, 1)  # small posterior variance rows
     mean_o, var_o = gp.predict(st, X)
@@ -344,11 +350,13 @@ def test_gp_predict_tensor_path(L, N, d, M, P):
 
 
 @pytest.mark.parametrize("N,d,M,P,ard,kind", [(300, 30, 3, 200, False, "matern"), (1000, 12, 2, 517, True, "matern"), (4096, 30, 3, 5000, False, "matern"),
-                                               (777, 22, 5, 1300, True, "rbf"), (513, 2, 1, 33, False, "rbf"), (2048, 24, 6, 4096, False, "matern")])
+                                               (777, 22, 5, 1300, True, "rbf"), (513, 2, 1, 33, False, "rbf"), (2048, 24, 6, 4096, False, "matern"),
+                                               (900, 48, 2, 700, False, "matern"), (600, 16, 7, 900, True, "rbf")])
 def test_gp_mean_only_kernel(L, N, d, M, P, ard, kind):
     """Predicts without variance (GPR_Matern.evaluate, once per generation in MOASMO.optimize) take gp_mean_direct_kernel:
     K_* is never written, kernel values in fp32, float64 partial sums.  Against the oracle: 1e-5 of max(|mean|, y_std);
-    isotropic and per-dimension length scales, both kernels, ragged P and N, 1 .. 6 objectives."""
+    isotropic and per-dimension length scales, both kernels, ragged P and N, 1 .. 7 objectives.  d > 32 or M > 6 take the
+    stored K_* (kstar_tensor_kernel + mean_split_kernel) under the same bars."""
     rng = np.random.default_rng(N + P)
     xlb, xub = np.zeros(d), np.ones(d)
     Xtr = rng.random((N, d))
